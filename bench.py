@@ -55,7 +55,14 @@ def parse_args():
     ap.add_argument("--pairs", type=int, default=1_000_000, help="pairs per GPU")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--configs", default="C2_10k,C3,C4,C5", help="extra configs to report ('' = none)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the results of the last timed step to DIR/<name>.npy (see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
+    return args
 
 
 def measured_peaks():
@@ -140,7 +147,6 @@ def run_reference(args):
     if rank != 0:
         return
     from oracle import oracle as orc
-    orc.build()
     threads = orc.hardware_threads()
     vals, sample = [], None
     for it in range(args.warmup + args.steps):
@@ -185,6 +191,30 @@ def pinned_results(torch, Results, P, ops_cap):
              "yend": out_t["yend"].numpy().view(np.uint32), "ops_off": out_t["ops_off"].numpy().view(np.uint64),
              "ops": out_t["ops"].numpy(), "clip_len": out_t["clip_len"].numpy().view(np.uint32)}
     return Results(P, ops_cap, out=views), out_t
+
+
+DUMP_PAIRS, DUMP_OPS_PAIRS = 1 << 20, 4096  # 6 x 8 MB of per-pair fields + <= 10 MB of ops: < 64 MB in all
+
+
+def dump_outputs(out_dir, res, n_pairs):
+    """Write the results a caller of the timed path receives to out_dir/<name>.npy, so that two builds can be
+    compared output for output: score, xstart, xend, ystart, yend of every pair (of a seeded sample of DUMP_PAIRS
+    pairs when there are more; pair_index names them) and the operations of a seeded sample of DUMP_OPS_PAIRS pairs
+    (ops: one (code, clip length) row per operation, ops_count rows per pair of ops_pair_index).  The fields are
+    float64, which holds every int32 / uint32 exactly; op codes and clip lengths are small enough for float32."""
+    os.makedirs(out_dir, exist_ok=True)
+    rng = np.random.default_rng(0)
+    idx = np.arange(n_pairs) if n_pairs <= DUMP_PAIRS else np.sort(rng.choice(n_pairs, DUMP_PAIRS, replace=False))
+    arrays = {"pair_index": idx.astype(np.float64)}
+    for f in ("score", "xstart", "xend", "ystart", "yend"):
+        arrays[f] = getattr(res, f)[idx].astype(np.float64)
+    oidx = np.sort(rng.choice(n_pairs, min(n_pairs, DUMP_OPS_PAIRS), replace=False))
+    ops = [res.ops_of(int(p)) for p in oidx]
+    arrays["ops_pair_index"] = oidx.astype(np.float64)
+    arrays["ops_count"] = np.array([len(o) for o in ops], dtype=np.float64)
+    arrays["ops"] = np.array([op for o in ops for op in o], dtype=np.float32).reshape(-1, 2)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def check_sample(orc, mode_name, oscoring, batch, idx, res, threads):
@@ -320,7 +350,11 @@ def main():
         t[rank] = ms_total / steps
         dist.all_reduce(t)
         ms_ranks = [round(float(v), 4) for v in t.tolist()]
-    eng.fetch(None)
+    if args.dump_outputs and world == 1:
+        eng.fetch(results)  # the last timed step's results; the passes below run the batch again
+        dump_outputs(args.dump_outputs, results, P)
+    else:
+        eng.fetch(None)
     st = eng.stats
     launches_step = int(st.kernel_launches) + (1 if world > 1 else 0)  # + the segment-header kernel
     # kernel-level numbers over instrumented passes (engine CUDA events on the same stream)
@@ -342,10 +376,11 @@ def main():
         torch.cuda.synchronize()
         if rank == 0:
             from oracle import oracle as orc
-            orc.build()
             total_pairs = world * P
             allres, keep_all = pinned_results(torch, Results, total_pairs, 64 * total_pairs)
             n_got, _ = eng.gathered_fetch(b["all"].data_ptr(), seg, world, allres)
+            if args.dump_outputs:
+                dump_outputs(args.dump_outputs, allres, total_pairs)
             rng = np.random.default_rng(7)
             bad, checked = 0, 0
             for r in range(world):
@@ -415,7 +450,6 @@ def main():
         d2h = int(getattr(sharded, "d2h", 0))
         if rank == 0 and allres is not None:  # the e2e arm's own output, checked like the resident arm's
             from oracle import oracle as orc2
-            orc2.build()
             idx = np.arange(0, P, max(1, P // 128))[:128]
             sub = (batch[0], batch[1][idx], batch[2][idx], batch[3][idx], batch[4][idx])
             ref, ops, off, _ = orc2.align_batch("local", oracle_scoring(orc2), *sub, threads=min(16, orc2.hardware_threads()))
@@ -445,7 +479,6 @@ def main():
     want_cfgs = [c for c in args.configs.split(",") if c]
     if want_cfgs:
         from oracle import oracle as orc
-        orc.build()
         othreads = min(32, orc.hardware_threads())
         flush = torch.empty(256 << 20, dtype=torch.uint8, device="cuda")
 
@@ -606,7 +639,6 @@ def main():
         cpu = None
         if world == 1 and not args.no_cpu_baseline:
             from oracle import oracle as orc
-            orc.build()
             threads = orc.hardware_threads()
             g, n, t = cpu_sample(orc, threads, target_s=12.0)
             g1, n1, t1 = cpu_sample(orc, 1, target_s=4.0)
