@@ -27,7 +27,7 @@ W_8_20 = os.environ.get("B2A_W_8_20")  # warps per CTA of the 8x20 fill (default
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
          "-Xcompiler", "-fPIC", "-Xcompiler", "-fwrapv", "--expt-relaxed-constexpr"] + ([f"-DB2A_W_8_20={W_8_20}"] if W_8_20 else []) + KS_DEFS
-HEADERS = ["b2a_common.cuh", "b2a_coop.cuh", "b2a_fill.cuh", "b2a_walk.cuh", "b2a_kernels.cuh", "b2a_plan.h", "b2a_banded.cuh", "b2a_banded_strip.cuh",
+HEADERS = ["b2a_common.cuh", "b2a_coop.cuh", "b2a_fill.cuh", "b2a_fill_pair16.cuh", "b2a_walk.cuh", "b2a_kernels.cuh", "b2a_plan.h", "b2a_banded.cuh", "b2a_banded_strip.cuh",
            "b2a_fill_launch.h", os.path.join("..", "..", "include", "b200align.h")]
 
 
@@ -56,6 +56,12 @@ def build(force: bool = False, verbose: bool = False) -> str:
         src = os.path.join(CSRC, "b2a_fill_inst.cu")
         if force or _stale(o, hdrs + [src]):
             jobs.append([NVCC, *FLAGS, f"-DB2A_G={g}", f"-DB2A_R={r}", f"-DB2A_MINB={MIN_BLOCKS.get((g, r), 1)}", "-c", src, "-o", o])
+    # the pair-packed 1x16 fill: 3 CTAs per SM like the int32 1x16 kernel
+    p16o = os.path.join(OBJ, "fill_pair16.o")
+    objs.append(p16o)
+    p16src = os.path.join(CSRC, "b2a_fill_pair16.cu")
+    if force or _stale(p16o, hdrs + [p16src]):
+        jobs.append([NVCC, *FLAGS, f"-DB2A_MINB={MIN_BLOCKS[(1, 16)]}", "-c", p16src, "-o", p16o])
     eo = os.path.join(OBJ, "engine.o")
     objs.append(eo)
     esrc = os.path.join(CSRC, "b2a_engine.cu")

@@ -18,6 +18,7 @@
 #define B2A_DEFINE_WALK_KERNEL
 #include "../../include/b200align.h"
 #include "b2a_fill_launch.h"
+#include "b2a_fill_pair16.cuh"
 #include "b2a_kernels.cuh"
 #include "b2a_plan.h"
 #include "b2a_walk.cuh"
@@ -118,6 +119,10 @@ struct b2a_engine {
   std::vector<uint64_t> eff_xoff, eff_yoff;
   bool last_walk_warp = false;
   uint64_t tb_budget = 0;
+  bool pairpack = true;            // B2A_PAIRPACK=0: never the pair-packed 1x16 fill (development knob: compare both)
+  bool p16 = false;                // the staged batch runs the pair-packed fill (pair16_eligible)
+  int32_t p16_bias = 0;
+  uint32_t p16_stage = 0;          // its per-warp staging: y of both blocks
 
   // batch state
   bool staged = false, ran = false;
@@ -135,7 +140,7 @@ struct b2a_engine {
       d_rowm, d_tb, d_opsscratch, d_lut, d_codemap, d_ctl, d_score, d_xs, d_xe, d_ys, d_ye, d_nops,
       d_opssrc, d_clip, d_status, d_nops64, d_opsoff, d_opsdense, d_scan, d_records, d_prog, d_bcells, d_bstatus,
       d_bopsend, d_bslab, d_branges, d_broff, d_bfill, d_bfoff, d_hmoff, d_hmxy, d_hpoff, d_hpidx, d_raw, d_gnops,
-      d_gnops64, d_goff, d_bcols, d_bstrip, d_bsoff, d_belig;
+      d_gnops64, d_goff, d_bcols, d_bstrip, d_bsoff, d_belig, d_lut16;
   uint32_t* h_nops = nullptr;  // pinned staging of b2a_gathered_fetch
   uint64_t h_nops_cap = 0;
   cudaEvent_t ev[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
@@ -283,6 +288,7 @@ int32_t b2a_engine_create(b2a_engine** out, int32_t device_id) {
   if (const char* env = getenv("B2A_TAIL_SPLIT")) e->tail_split = atoi(env) != 0;
   if (const char* env = getenv("B2A_NO_PACKREL")) e->no_packrel = atoi(env) != 0;
   if (const char* env = getenv("B2A_SPLIT_TIMING")) e->split_timing = atoi(env) != 0;
+  if (const char* env = getenv("B2A_PAIRPACK")) e->pairpack = atoi(env) != 0;
   if (const char* env = getenv("B2A_WALK_CTA_WARPS")) {
     const int v = atoi(env);
     if (v == 1 || v == 2 || v == 4 || v == 8 || v == 16 || v == 32) e->walk_cta_warps = (uint32_t)v;
@@ -326,7 +332,7 @@ int32_t b2a_engine_destroy(b2a_engine* e) {
                     &e->d_nops64, &e->d_opsoff, &e->d_opsdense, &e->d_scan, &e->d_records, &e->d_prog, &e->d_bcells,
                     &e->d_bstatus, &e->d_bopsend, &e->d_bslab, &e->d_branges, &e->d_broff, &e->d_bfill, &e->d_hmoff, &e->d_hmxy,
                     &e->d_hpoff, &e->d_hpidx, &e->d_raw, &e->d_gnops, &e->d_gnops64, &e->d_goff,
-                    &e->d_bfoff, &e->d_bcols, &e->d_bstrip, &e->d_bsoff, &e->d_belig};
+                    &e->d_bfoff, &e->d_bcols, &e->d_bstrip, &e->d_bsoff, &e->d_belig, &e->d_lut16};
   for (DevBuf* b : bufs) b->release();
   for (auto& v : e->ev)
     if (v) cudaEventDestroy(v);
@@ -581,6 +587,37 @@ static int32_t compact_ops(b2a_engine* e, uint64_t scratch_bytes, cudaStream_t s
   return B2A_OK;
 }
 
+// The pair-packed fill (b2a_fill_pair16.cuh) carries every value in 16 bits: it runs a wave of the 1x16 local
+// fill only when the wave is one shape small enough for that.  Returns the bias of its score domain, or -1.
+static int32_t pair16_eligible(const b2a_engine* e, const Plan& pl, int G, int R) {
+  const DevScoring& sc = e->sc;
+  if (!e->pairpack || G != 1 || R != 16 || e->flags != P16_FLAGS) return -1;
+  if (sc.alpha < 1 || sc.alpha > P16_MAX_ALPHA || pl.maxm > 256 || pl.maxn > 255 || pl.blocks.empty()) return -1;
+  for (uint64_t i = 0; i < pl.n_pairs; ++i)  // one shape: the two blocks of a task share their loop bounds
+    if (pl.pm[i] != pl.maxm || pl.pn[i] != pl.maxn) return -1;
+  int32_t lo = e->lut_host[0], hi = e->lut_host[0];
+  for (int k = 0; k < sc.alpha * sc.alpha; ++k) {
+    lo = std::min(lo, e->lut_host[k]);
+    hi = std::max(hi, e->lut_host[k]);
+  }
+  // a local score never exceeds min(m, n) substitutions at the best score: the tracker keys hold it in 8 bits
+  if ((int64_t)std::min(pl.maxm, pl.maxn) * std::max(hi, 0) > 255) return -1;
+  if (sc.gap_open < -2048 || sc.gap_extend < -2048 || lo < -2048) return -1;  // stored values stay below 2^14
+  return 4 * std::max(std::max(-sc.gap_open, -lo), 0);
+}
+
+// K1 of a wave (or a part of one): the pair-packed fill when the batch was staged for it, else the int32 shape
+static cudaError_t launch_fill(b2a_engine* e, const FillParams& fp, uint32_t ntasks, cudaStream_t st, int* grid_out,
+                               int dry) {
+  if (e->p16) {
+    FillParams f = fp;
+    f.lut = e->d_lut16.as<int32_t>();
+    f.smem_seq_bytes = e->p16_stage;
+    return launch_fill_pair16(f, e->p16_bias, e->num_sms, st, grid_out, dry);
+  }
+  return e->shape->launch(e->flags, fp, ntasks, e->num_sms, st, grid_out, dry);
+}
+
 extern "C" {
 
 int32_t b2a_batch_stage(b2a_engine* e, int32_t mode, const b2a_scoring* s, const b2a_pairs* pairs) {
@@ -622,6 +659,16 @@ int32_t b2a_batch_stage(b2a_engine* e, int32_t mode, const b2a_scoring* s, const
     R = (pad16 * 100 <= pad8 * 112) ? 16 : 8;
   }
   const Plan& pl = e->plan;
+  const int32_t p16_bias = pair16_eligible(e, pl, G, R);
+  e->p16 = p16_bias >= 0;
+  e->p16_bias = e->p16 ? p16_bias : 0;
+  e->p16_stage = e->p16 ? 2 * pl.blocks[0].ywords * 32 * 4 : 0;
+  std::vector<int32_t> lut16;
+  if (e->p16) {
+    lut16.resize((size_t)p16_lut_entries(sc.alpha));
+    p16_build_lut(e->lut_host.data() + (size_t)sc.alpha * sc.alpha, sc.alpha, lut16.data());
+    CK(e->d_lut16.reserve(lut16.size() * 4 + 16));
+  }
 
   // device memory
   CK(e->d_xoff.reserve(n * 8 + 8));
@@ -664,7 +711,7 @@ int32_t b2a_batch_stage(b2a_engine* e, int32_t mode, const b2a_scoring* s, const
   }
   {
     const size_t blocks_bytes = pl.blocks.size() * sizeof(Block), lut_b = e->lut_host.size() * 4;
-    const size_t need = 3 * n * 4 + blocks_bytes + 256 + lut_b + 64;
+    const size_t need = 3 * n * 4 + blocks_bytes + 256 + lut_b + lut16.size() * 4 + 80;
     if (e->h_plan_cap < need) {
       if (e->h_plan) cudaFreeHost(e->h_plan);
       e->h_plan = nullptr;
@@ -686,6 +733,7 @@ int32_t b2a_batch_stage(b2a_engine* e, int32_t mode, const b2a_scoring* s, const
     CK(up_staged(e->d_blocks, pl.blocks.data(), blocks_bytes));
     CK(up_staged(e->d_codemap, e->codemap_host, 256));
     if (lut_b) CK(up_staged(e->d_lut, e->lut_host.data(), lut_b));
+    if (!lut16.empty()) CK(up_staged(e->d_lut16, lut16.data(), lut16.size() * 4));
   }
   // the caller's arrays are read by the copies above: wait for them unless the caller (the chunk pipeline of
   // b2a_align_batch) keeps them alive itself
@@ -823,10 +871,10 @@ int32_t b2a_batch_run(b2a_engine* e) {
     // remainder (B) are filled back to back, and K2 of A runs beside the fill of B: B's few CTAs go out on the
     // high-priority stream first, A's walk takes the rest of the GPU.
     uint32_t split_b = 0;  // blocks of part A (0: no split)
-    if (e->tail_split && !overlap && pl.waves.size() == 1 && warp_walk && pl.G != 32 && !use_tail && e->walk_mode != 1 &&
+    if (e->tail_split && !e->p16 && !overlap && pl.waves.size() == 1 && warp_walk && pl.G != 32 && !use_tail && e->walk_mode != 1 &&
         fp.task_limit == 0) {
       int resident = 0;
-      CK(e->shape->launch(e->flags, fp, fill_tasks, e->num_sms, st, &resident, 1));
+      CK(launch_fill(e, fp, fill_tasks, st, &resident, 1));
       const uint32_t slots = (uint32_t)resident, tasks = fill_tasks;
       if (slots > 0 && tasks > slots) {
         const uint32_t rounds = tasks / slots, rem = tasks % slots;
@@ -861,7 +909,7 @@ int32_t b2a_batch_run(b2a_engine* e) {
       if (e->split_timing && !e->split_ev[0])
         for (auto& v : e->split_ev) CK(cudaEventCreate(&v));
       if (e->split_timing) CK(cudaEventRecord(e->split_ev[0], st));
-      CK(e->shape->launch(e->flags, fa, fa.nblocks * (uint32_t)pl.G, e->num_sms, st, &e->last_grid, 0));
+      CK(launch_fill(e, fa, fa.nblocks * (uint32_t)pl.G, st, &e->last_grid, 0));
       if (e->split_timing) CK(cudaEventRecord(e->split_ev[1], st));
       CK(cudaEventRecord(e->sub_ev[0], st));  // fill A done
       // fill B + walk B on the high-priority stream, walk A on the auxiliary one
@@ -871,7 +919,7 @@ int32_t b2a_batch_run(b2a_engine* e) {
       cudaStream_t sB = e->tail_stream, sA = e->aux_stream;
       CK(cudaStreamWaitEvent(sB, e->sub_ev[0], 0));
       CK(cudaStreamWaitEvent(sA, e->sub_ev[0], 0));
-      CK(e->shape->launch(e->flags, fb, fb.nblocks * (uint32_t)pl.G, e->num_sms, sB, nullptr, 0));
+      CK(launch_fill(e, fb, fb.nblocks * (uint32_t)pl.G, sB, nullptr, 0));
       CK(cudaEventRecord(e->wave_ev[3 * wi + 1], sB));  // every fill has finished
       if (e->split_timing) CK(cudaEventRecord(e->split_ev[2], sB));
       walk_warp_kernel<<<wa.nblocks * 32 / wcta_warps, wcta_warps * 32, (size_t)per_warp_smem * wcta_warps, sA>>>(wa);
@@ -918,7 +966,7 @@ int32_t b2a_batch_run(b2a_engine* e) {
         f2.nblocks = hi_b - lo_b;
         f2.task_counter = ctl + 8 + sidx;
         f2.task_limit = 1;  // CTAs retire after one task per warp: the walks' CTAs get onto the SMs in between
-        CK(e->shape->launch(e->flags, f2, f2.nblocks * (uint32_t)pl.G, e->num_sms, fs, &e->last_grid, 0));
+        CK(launch_fill(e, f2, f2.nblocks * (uint32_t)pl.G, fs, &e->last_grid, 0));
         ++e->launches;
         CK(cudaEventRecord(e->sub_ev[sidx], fs));
         CK(cudaStreamWaitEvent(e->tail_stream, e->sub_ev[sidx], 0));
@@ -939,7 +987,7 @@ int32_t b2a_batch_run(b2a_engine* e) {
       continue;
     }
     CK(cudaEventRecord(e->wave_ev[3 * wi + 0], st));
-    CK(e->shape->launch(e->flags, fp, fill_tasks, e->num_sms, st, &e->last_grid, 0));
+    CK(launch_fill(e, fp, fill_tasks, st, &e->last_grid, 0));
     ++e->launches;
     CK(cudaEventRecord(e->wave_ev[3 * wi + 1], st));
     if (use_tail) {  // K2 and everything after it on the high-priority stream
