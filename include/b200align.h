@@ -186,6 +186,25 @@ int32_t b2a_engine_set_pipeline(b2a_engine* e, int32_t chunks);
 int32_t b2a_align_batch(b2a_engine* e, int32_t mode, const b2a_scoring* scoring,
                         const b2a_pairs* pairs, b2a_results* results, b2a_stats* stats);
 
+/* Score-only outputs: the score, xend and yend of the Alignment b2a_align_batch would return (caller-allocated
+ * host arrays; any of them may be NULL). */
+typedef struct b2a_score_results {
+  int32_t* score;   /* [n_pairs] */
+  uint32_t* xend;   /* [n_pairs] */
+  uint32_t* yend;   /* [n_pairs] */
+  uint32_t* status; /* [n_pairs] B2A_PAIR_* or NULL, same contract as b2a_results.status */
+} b2a_score_results;
+
+/* Score-only form of b2a_align_batch, for callers that rank or filter candidates and never read the path: the
+ * fill keeps no traceback (stats.traceback_bytes == 0, one wave whatever the traceback budget), and K2 computes
+ * row m and the last-column fix-ups, then walks only row m and column n -- the only cells whose moves change xend
+ * and yend.  score, xend and yend are bit-identical to b2a_align_batch's for every pair that call reports as
+ * B2A_PAIR_OK; xstart, ystart and ops are not produced.  Validation, errors, shape choice and the chunk pipeline of
+ * batches >= 262,144 pairs are b2a_align_batch's.  A reference panic is seen only where that walk meets it: a pair
+ * whose corrupt move lies deeper inside the matrix keeps its score with status B2A_PAIR_OK here. */
+int32_t b2a_score_batch(b2a_engine* e, int32_t mode, const b2a_scoring* scoring, const b2a_pairs* pairs,
+                        b2a_score_results* results, b2a_stats* stats);
+
 /* Packed input (SURVEY 8f rank 2): the sequences as bio::data_structures::bitenc::BitEnc storage
  * (src/data_structures/bitenc.rs:50-56: 32-bit blocks, `width` bits per symbol, 32 - 32 % width usable bits per
  * block; symbol i sits at bit (i*width) % usable of block (i*width) / usable, bitenc.rs:319-338), holding the ranks

@@ -24,7 +24,7 @@ ABI_SYMBOLS = [
     "b2a_engine_create", "b2a_engine_destroy", "b2a_last_error", "b2a_version",
     "b2a_engine_set_stream", "b2a_engine_set_traceback_budget", "b2a_engine_set_tuning",
     "b2a_engine_set_pipeline", "b2a_engine_set_walk", "b2a_engine_last_alphabet",
-    "b2a_align_batch", "b2a_align_batch_banded", "b2a_align_batch_banded_hinted", "b2a_banded_band_ranges", "b2a_banded_strip_pairs", "b2a_batch_stage", "b2a_batch_run",
+    "b2a_align_batch", "b2a_score_batch", "b2a_align_batch_banded", "b2a_align_batch_banded_hinted", "b2a_banded_band_ranges", "b2a_banded_strip_pairs", "b2a_batch_stage", "b2a_batch_run",
     "b2a_batch_fetch", "b2a_batch_records", "b2a_batch_records_into", "b2a_record_stride",
     "b2a_records_decode", "b2a_batch_compact_bytes", "b2a_batch_compact_into", "b2a_compact_decode",
     "b2a_batch_compact_fixed", "b2a_gathered_fetch", "b2a_align_batch_packed", "b2a_align_batch_banded_packed",
@@ -66,6 +66,11 @@ class CResults(C.Structure):
                 ("ystart", C.c_void_p), ("yend", C.c_void_p), ("ops_off", C.c_void_p),
                 ("ops", C.c_void_p), ("ops_capacity", C.c_uint64), ("clip_len", C.c_void_p),
                 ("status", C.c_void_p)]
+
+
+class CScoreResults(C.Structure):
+    """b2a_score_results (include/b200align.h)"""
+    _fields_ = [("score", C.c_void_p), ("xend", C.c_void_p), ("yend", C.c_void_p), ("status", C.c_void_p)]
 
 
 class CStats(C.Structure):
@@ -110,6 +115,8 @@ def load():
     L.b2a_engine_last_alphabet.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(C.c_uint32)]
     L.b2a_align_batch.argtypes = [C.c_void_p, C.c_int32, C.POINTER(CScoring), C.POINTER(CPairs),
                                   C.POINTER(CResults), C.POINTER(CStats)]
+    L.b2a_score_batch.argtypes = [C.c_void_p, C.c_int32, C.POINTER(CScoring), C.POINTER(CPairs),
+                                  C.POINTER(CScoreResults), C.POINTER(CStats)]
     L.b2a_align_batch_banded.argtypes = [C.c_void_p, C.c_int32, C.POINTER(CScoring), C.c_uint32,
                                          C.c_uint32, C.POINTER(CPairs), C.POINTER(CResults),
                                          C.POINTER(CStats)]

@@ -80,6 +80,8 @@ enum : int {
   F_PACKREL = 128,   // long sequences (m or n > 4095, |S| < 2^18): the same packed keys with RELATIVE indices -- the row
                      // tracker's column inside a chunk of 2^KREL_BITS columns (flushed to the rows arena at each chunk
                      // end), the column tracker's row inside the strip (made absolute where the strip hands it on)
+  F_NOTB = 256,      // score-only batch (b2a_score_batch): no interior traceback -- no nibble accumulators, no stores to
+                     // the traceback arena; the boundary row, rows arena and row m-1 stay word for word the same
 };
 #ifndef B2A_KREL_BITS
 #define B2A_KREL_BITS 12  // (a test build shortens the chunks to exercise the flushes on small inputs)

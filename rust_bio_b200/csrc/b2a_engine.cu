@@ -126,6 +126,7 @@ struct b2a_engine {
 
   // batch state
   bool staged = false, ran = false;
+  bool score_only = false;         // the staged batch is a score-only one (b2a_score_batch): F_NOTB fill, score-only K2
   Plan plan;
   DevScoring sc{};
   int flags = 0, mode = 0;
@@ -394,6 +395,7 @@ static int32_t stage_front(b2a_engine* e, int32_t mode, const b2a_scoring* s, co
                            uint32_t& maxm, uint32_t& maxn, int64_t& score_bound) {
   if (!e || !s || !pairs) return B2A_E_INVALID;
   e->staged = e->ran = false;
+  e->score_only = false;
   if (mode < 0 || mode > 3) return e->fail(B2A_E_INVALID, "mode must be B2A_MODE_*");
   int rc = validate_scoring(e, s);
   if (rc) return rc;
@@ -613,19 +615,20 @@ static cudaError_t launch_fill(b2a_engine* e, const FillParams& fp, uint32_t nta
     FillParams f = fp;
     f.lut = e->d_lut16.as<int32_t>();
     f.smem_seq_bytes = e->p16_stage;
-    return launch_fill_pair16(f, e->p16_bias, e->num_sms, st, grid_out, dry);
+    return launch_fill_pair16(f, e->p16_bias, e->score_only, e->num_sms, st, grid_out, dry);
   }
-  return e->shape->launch(e->flags, fp, ntasks, e->num_sms, st, grid_out, dry);
+  return e->shape->launch(e->flags | (e->score_only ? F_NOTB : 0), fp, ntasks, e->num_sms, st, grid_out, dry);
 }
 
-extern "C" {
-
-int32_t b2a_batch_stage(b2a_engine* e, int32_t mode, const b2a_scoring* s, const b2a_pairs* pairs) {
+// Stage a batch for b2a_batch_run: the full batch, or (score_only) the score-only one of b2a_score_batch, which
+// fills without the traceback (one wave, no traceback arena) and runs the score-only K2 without ops.
+static int32_t batch_stage(b2a_engine* e, int32_t mode, const b2a_scoring* s, const b2a_pairs* pairs, bool score_only) {
   if (!e || !s || !pairs) return B2A_E_INVALID;
   uint32_t maxm = 0, maxn = 0;
   int64_t score_bound = 0;
   int rc = stage_front(e, mode, s, pairs, maxm, maxn, score_bound);
   if (rc) return rc;
+  e->score_only = score_only;
   const uint64_t n = e->n_pairs;
   const DevScoring sc = e->sc;
   cudaStream_t st = e->stream;
@@ -646,7 +649,7 @@ int32_t b2a_batch_stage(b2a_engine* e, int32_t mode, const b2a_scoring* s, const
   for (int attempt = 0;; ++attempt) {
     e->shape = find_shape(G, R);
     if (!e->shape) return e->fail(B2A_E_INVALID, "no fill kernel for the requested shape");
-    build_plan(e->plan, pairs->x_len, pairs->y_len, n, G, R, budget);
+    build_plan(e->plan, pairs->x_len, pairs->y_len, n, G, R, budget, score_only);
     if (64 + lut_bytes + (uint64_t)fill_warps_of(G, R) * e->plan.smem_seq_bytes <= kMaxStageSmem) break;
     // Shapes with several pairs per warp stage 32/G whole (x, y) per warp; long sequences (a read against a
     // 15 kb reference ...) only fit the warp-per-pair shape, which stages one strip of x and one y per warp
@@ -685,20 +688,22 @@ int32_t b2a_batch_stage(b2a_engine* e, int32_t mode, const b2a_scoring* s, const
   CK(e->d_rowm.reserve(pl.max_rowm + 16));
   CK(e->d_tb.reserve(pl.max_tb + 16));
   CK(e->d_prog.reserve(pl.max_strip_tasks * 4 + 16));
-  CK(e->d_opsscratch.reserve(pl.ops_bytes + 16));
   CK(e->d_lut.reserve(e->lut_host.size() * 4 + 16));
   CK(e->d_codemap.reserve(256));
   CK(e->d_score.reserve(n * 4 + 4));
-  CK(e->d_xs.reserve(n * 4 + 4));
   CK(e->d_xe.reserve(n * 4 + 4));
-  CK(e->d_ys.reserve(n * 4 + 4));
   CK(e->d_ye.reserve(n * 4 + 4));
-  CK(e->d_nops.reserve(n * 4 + 4));
-  CK(e->d_opssrc.reserve(n * 8 + 8));
-  CK(e->d_clip.reserve(n * 16 + 16));
   CK(e->d_status.reserve(n * 4 + 4));
-  CK(e->d_nops64.reserve((n + 1) * 8));
-  CK(e->d_opsoff.reserve((n + 1) * 8));
+  if (!score_only) {  // the ops and the start coordinates of the full path
+    CK(e->d_opsscratch.reserve(pl.ops_bytes + 16));
+    CK(e->d_xs.reserve(n * 4 + 4));
+    CK(e->d_ys.reserve(n * 4 + 4));
+    CK(e->d_nops.reserve(n * 4 + 4));
+    CK(e->d_opssrc.reserve(n * 8 + 8));
+    CK(e->d_clip.reserve(n * 16 + 16));
+    CK(e->d_nops64.reserve((n + 1) * 8));
+    CK(e->d_opsoff.reserve((n + 1) * 8));
+  }
 
   // host -> device.  The plan vectors go through a pinned staging arena so that their copies are truly
   // asynchronous (a copy from pageable memory first waits for the stream: it would serialise the host with the
@@ -740,6 +745,12 @@ int32_t b2a_batch_stage(b2a_engine* e, int32_t mode, const b2a_scoring* s, const
   if (!e->stage_nosync) CK(cudaStreamSynchronize(st));
   e->staged = true;
   return B2A_OK;
+}
+
+extern "C" {
+
+int32_t b2a_batch_stage(b2a_engine* e, int32_t mode, const b2a_scoring* s, const b2a_pairs* pairs) {
+  return batch_stage(e, mode, s, pairs, false);
 }
 
 int32_t b2a_batch_run(b2a_engine* e) {
@@ -838,6 +849,9 @@ int32_t b2a_batch_run(b2a_engine* e) {
     // (running K2 inside K1's warps was measured: 28.4 ms vs 22.4 + 3.2 ms separately -- the latency-bound
     //  walk holds one of only 12 resident warps per SM; K2 stays its own launch)
     const bool fuse = false;
+    // K2 in its two forms: the walk, or the score-only epilogue (row m, fix-ups, end walk) of a score-only batch
+    void (*const k2_warp)(const WalkParams) = e->score_only ? score_warp_kernel : walk_warp_kernel;
+    void (*const k2_lane)(const WalkParams) = e->score_only ? score_kernel : walk_kernel;
     fp.task_limit = (pl.G == 32) ? 0u : e->fill_task_limit;  // strip-pipelined tasks need the persistent grid
     const uint64_t wave_pairs = (uint64_t)nb * 32;
     const bool warp_walk = e->walk_mode == 2 || (e->walk_mode == 0 && wave_pairs <= kWarpWalkMaxPairs);
@@ -852,7 +866,7 @@ int32_t b2a_batch_run(b2a_engine* e) {
       if (!wcta_warps) wcta_warps = (uint64_t)per_warp * 8 <= 96 * 1024 ? 8u : 4u;
       per_warp_smem = (uint64_t)per_warp * wcta_warps <= 96 * 1024 ? per_warp : 0u;
       if ((size_t)per_warp_smem * wcta_warps > 48 * 1024)
-        CK(cudaFuncSetAttribute(walk_warp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(per_warp_smem * wcta_warps)));
+        CK(cudaFuncSetAttribute(k2_warp, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(per_warp_smem * wcta_warps)));
     }
     if (!wcta_warps) wcta_warps = 4;
     wp.seq_smem_per_warp = per_warp_smem;
@@ -922,10 +936,10 @@ int32_t b2a_batch_run(b2a_engine* e) {
       CK(launch_fill(e, fb, fb.nblocks * (uint32_t)pl.G, sB, nullptr, 0));
       CK(cudaEventRecord(e->wave_ev[3 * wi + 1], sB));  // every fill has finished
       if (e->split_timing) CK(cudaEventRecord(e->split_ev[2], sB));
-      walk_warp_kernel<<<wa.nblocks * 32 / wcta_warps, wcta_warps * 32, (size_t)per_warp_smem * wcta_warps, sA>>>(wa);
+      k2_warp<<<wa.nblocks * 32 / wcta_warps, wcta_warps * 32, (size_t)per_warp_smem * wcta_warps, sA>>>(wa);
       CK(cudaGetLastError());
       if (e->split_timing) CK(cudaEventRecord(e->split_ev[3], sA));
-      walk_warp_kernel<<<wb.nblocks * 32 / wcta_warps, wcta_warps * 32, (size_t)per_warp_smem * wcta_warps, sB>>>(wb);
+      k2_warp<<<wb.nblocks * 32 / wcta_warps, wcta_warps * 32, (size_t)per_warp_smem * wcta_warps, sB>>>(wb);
       CK(cudaGetLastError());
       if (e->split_timing) CK(cudaEventRecord(e->split_ev[4], sB));
       e->split_ran = true;
@@ -974,8 +988,8 @@ int32_t b2a_batch_run(b2a_engine* e) {
         WalkParams w2 = wp;
         w2.blocks = wp.blocks + lo_b;
         w2.nblocks = hi_b - lo_b;
-        if (warp_walk) walk_warp_kernel<<<w2.nblocks * 32 / wcta_warps, wcta_warps * 32, (size_t)per_warp_smem * wcta_warps, e->tail_stream>>>(w2);
-        else walk_kernel<<<(w2.nblocks * 32 + 127) / 128, 128, 0, e->tail_stream>>>(w2);
+        if (warp_walk) k2_warp<<<w2.nblocks * 32 / wcta_warps, wcta_warps * 32, (size_t)per_warp_smem * wcta_warps, e->tail_stream>>>(w2);
+        else k2_lane<<<(w2.nblocks * 32 + 127) / 128, 128, 0, e->tail_stream>>>(w2);
         CK(cudaGetLastError());
         ++e->launches;
       }
@@ -1000,10 +1014,10 @@ int32_t b2a_batch_run(b2a_engine* e) {
       // pairs share every cache line); one WARP per pair cuts the per-pair latency chain (prefix-maximum passes,
       // prefetched walk) and is what small / medium batches and long sequences need (b2a_walk.cuh).
       if (warp_walk) {
-        walk_warp_kernel<<<nb * 32 / wcta_warps, wcta_warps * 32, (size_t)per_warp_smem * wcta_warps, st>>>(wp);  // 32 warps (pairs) per block of the plan
+        k2_warp<<<nb * 32 / wcta_warps, wcta_warps * 32, (size_t)per_warp_smem * wcta_warps, st>>>(wp);  // 32 warps (pairs) per block of the plan
       } else {
         const unsigned wgrid = (nb * 32 + 127) / 128;
-        walk_kernel<<<wgrid, 128, 0, st>>>(wp);
+        k2_lane<<<wgrid, 128, 0, st>>>(wp);
       }
       CK(cudaGetLastError());
       ++e->launches;
@@ -1013,7 +1027,7 @@ int32_t b2a_batch_run(b2a_engine* e) {
     ++wi;
   }
   CK(cudaEventRecord(e->ev[4], st));
-  {
+  if (!e->score_only) {
     int rc2 = compact_ops(e, pl.ops_bytes, st);
     if (rc2) return rc2;
   }
@@ -1127,14 +1141,19 @@ static void collect_stats(b2a_engine* e, b2a_stats* stats) {
 }
 
 // finish one pipeline slot: its chunk's results are complete on the device; place its ops after `base`
-static int32_t slot_finish(b2a_engine* e, b2a_engine::PipeSlot& sl, b2a_results* r, uint64_t& base,
-                           b2a_stats* agg) {
+// (r == null: a score-only chunk, `status` is its caller's status array)
+static int32_t slot_finish(b2a_engine* e, b2a_engine::PipeSlot& sl, b2a_results* r, const uint32_t* status,
+                           uint64_t& base, b2a_stats* agg) {
   b2a_engine* c = sl.eng;
   sl.busy = false;
   cudaError_t ce = cudaStreamSynchronize(c->res_stream());
   if (ce != cudaSuccess) return e->cuda_fail("pipeline: cudaStreamSynchronize", ce);
   if (sl.h_ctl[0]) return e->fail(B2A_E_INVALID, "a sequence byte is outside the scoring alphabet");
-  if (sl.h_ctl[1] && !r->status) return e->fail(B2A_E_RANGE, "traceback walk met an impossible move (reference panics at mod.rs:905)");
+  if (sl.h_ctl[1] && !status) return e->fail(B2A_E_RANGE, "traceback walk met an impossible move (reference panics at mod.rs:905)");
+  if (!r) {
+    collect_stats(c, agg);
+    return B2A_OK;
+  }
   const uint64_t total = sl.h_opsoff[sl.n];
   if (r->ops) {
     if (base + total > r->ops_capacity) return e->fail(B2A_E_CAPACITY, "ops buffer too small for this batch");
@@ -1153,9 +1172,14 @@ static int32_t slot_finish(b2a_engine* e, b2a_engine::PipeSlot& sl, b2a_results*
   return B2A_OK;
 }
 
+static int32_t score_fetch(b2a_engine* e, b2a_score_results* r, b2a_stats* stats);
+
+// The chunk pipeline of a large batch: full results into r, or (r == null) score-only results into sr
 static int32_t align_batch_pipelined(b2a_engine* e, int32_t mode, const b2a_scoring* scoring,
-                                     const b2a_pairs* pairs, b2a_results* r, b2a_stats* stats) {
+                                     const b2a_pairs* pairs, b2a_results* r, b2a_score_results* sr, b2a_stats* stats) {
   const uint64_t n = pairs->n_pairs;
+  const bool score_only = r == nullptr;
+  const uint32_t* status = score_only ? sr->status : r->status;
   // chunk boundaries: K chunks, the first and the last half as large as the middle ones (the GPU idles
   // while the first chunk is staged and the host idles while the last one drains)
   uint64_t K = (uint64_t)e->pipe_chunks;
@@ -1208,7 +1232,7 @@ static int32_t align_batch_pipelined(b2a_engine* e, int32_t mode, const b2a_scor
     const uint64_t lo = cut[c], hi = cut[c + 1], nc = hi - lo;
     b2a_engine::PipeSlot& sl = e->slots[c % b2a_engine::kSlots];
     if (sl.busy) {
-      rc = slot_finish(e, sl, r, base, &agg);
+      rc = slot_finish(e, sl, r, status, base, &agg);
       if (rc) break;
     }
     if (!sl.eng) {
@@ -1308,7 +1332,7 @@ static int32_t align_batch_pipelined(b2a_engine* e, int32_t mode, const b2a_scor
       sc_chunk.alphabet = inferred.data();
       sc_chunk.alphabet_len = (uint32_t)inferred.size();
     }
-    rc = b2a_batch_stage(ch, mode, &sc_chunk, &sub);
+    rc = batch_stage(ch, mode, &sc_chunk, &sub, score_only);
     if (rc == B2A_OK && c == 0 && !(scoring->alphabet && scoring->alphabet_len)) inferred = ch->last_syms;
     const double tc2 = now();
     if (rc == B2A_OK) rc = b2a_batch_run(ch);
@@ -1327,6 +1351,20 @@ static int32_t align_batch_pipelined(b2a_engine* e, int32_t mode, const b2a_scor
       return cudaMemcpyAsync(dst, bf.p, bytes, cudaMemcpyDeviceToHost, st);
     };
     cudaError_t ce = cudaMemcpyAsync(sl.h_ctl, ch->d_ctl.p, 8, cudaMemcpyDeviceToHost, st);
+    if (score_only) {
+      if (ce == cudaSuccess) ce = down(sr->score ? sr->score + lo : nullptr, ch->d_score, nc * 4);
+      if (ce == cudaSuccess) ce = down(sr->xend ? sr->xend + lo : nullptr, ch->d_xe, nc * 4);
+      if (ce == cudaSuccess) ce = down(sr->yend ? sr->yend + lo : nullptr, ch->d_ye, nc * 4);
+      if (ce == cudaSuccess) ce = down(sr->status ? sr->status + lo : nullptr, ch->d_status, nc * 4);
+      if (ce != cudaSuccess) {
+        rc = e->cuda_fail("pipeline: result D2H", ce);
+        break;
+      }
+      sl.lo = lo;
+      sl.n = nc;
+      sl.busy = true;
+      continue;
+    }
     if (ce == cudaSuccess) ce = down(r->score ? r->score + lo : nullptr, ch->d_score, nc * 4);
     if (ce == cudaSuccess) ce = down(r->xstart ? r->xstart + lo : nullptr, ch->d_xs, nc * 4);
     if (ce == cudaSuccess) ce = down(r->xend ? r->xend + lo : nullptr, ch->d_xe, nc * 4);
@@ -1352,7 +1390,7 @@ static int32_t align_batch_pipelined(b2a_engine* e, int32_t mode, const b2a_scor
     if (!pick) break;
     b2a_engine::PipeSlot& sl = *pick;
     if (rc == B2A_OK) {
-      rc = slot_finish(e, sl, r, base, &agg);
+      rc = slot_finish(e, sl, r, status, base, &agg);
     } else {
       cudaStreamSynchronize(sl.eng->stream);
       cudaStreamSynchronize(sl.eng->res_stream());
@@ -1361,13 +1399,13 @@ static int32_t align_batch_pipelined(b2a_engine* e, int32_t mode, const b2a_scor
   }
   if (rc == B2A_E_INVALID && !inferred.empty() && e->err.find("alphabet") != std::string::npos) {
     // a later chunk held a byte the first chunk did not: redo the batch without the optimistic reuse
-    int32_t r2 = b2a_batch_stage(e, mode, scoring, pairs);
+    int32_t r2 = batch_stage(e, mode, scoring, pairs, score_only);
     if (r2 == B2A_OK) r2 = b2a_batch_run(e);
-    if (r2 == B2A_OK) r2 = b2a_batch_fetch(e, r, stats);
+    if (r2 == B2A_OK) r2 = score_only ? score_fetch(e, sr, stats) : b2a_batch_fetch(e, r, stats);
     return r2;
   }
   if (rc) return rc;
-  if (r->ops_off) r->ops_off[n] = base;
+  if (!score_only && r->ops_off) r->ops_off[n] = base;
   if (stats) *stats = agg;
   return B2A_OK;
 }
@@ -1379,13 +1417,65 @@ int32_t b2a_align_batch(b2a_engine* e, int32_t mode, const b2a_scoring* scoring,
   if (e->pipe_chunks >= 2 && results && pairs->n_pairs >= 262144) {
     e->staged = e->ran = false;
     if (cudaSetDevice(e->device) != cudaSuccess) return e->fail(B2A_E_NO_DEVICE, "cudaSetDevice failed");
-    return align_batch_pipelined(e, mode, scoring, pairs, results, stats);
+    return align_batch_pipelined(e, mode, scoring, pairs, results, nullptr, stats);
   }
   int rc = b2a_batch_stage(e, mode, scoring, pairs);
   if (rc) return rc;
   rc = b2a_batch_run(e);
   if (rc) return rc;
   return b2a_batch_fetch(e, results, stats);
+}
+
+}  // extern "C"
+
+// results of a score-only batch that b2a_batch_run has run
+static int32_t score_fetch(b2a_engine* e, b2a_score_results* r, b2a_stats* stats) {
+  cudaStream_t st = e->res_stream();
+  const uint64_t n = e->n_pairs;
+  uint64_t d2h = 0;
+  uint32_t ctl[2] = {0, 0};
+  CK(cudaMemcpyAsync(ctl, e->d_ctl.p, 8, cudaMemcpyDeviceToHost, st));
+  if (r && n) {
+    auto down = [&](void* dst, const DevBuf& b, size_t bytes) -> cudaError_t {
+      if (!dst || !bytes) return cudaSuccess;
+      d2h += bytes;
+      return cudaMemcpyAsync(dst, b.p, bytes, cudaMemcpyDeviceToHost, st);
+    };
+    CK(down(r->score, e->d_score, n * 4));
+    CK(down(r->xend, e->d_xe, n * 4));
+    CK(down(r->yend, e->d_ye, n * 4));
+    CK(down(r->status, e->d_status, n * 4));
+  }
+  CK(cudaStreamSynchronize(st));
+  if (ctl[0]) return e->fail(B2A_E_INVALID, "a sequence byte is outside the scoring alphabet");
+  if (ctl[1] && !(r && r->status))
+    return e->fail(B2A_E_RANGE, "traceback walk met an impossible move (the reference panics here: mod.rs:905)");
+  if (stats) {
+    std::memset(stats, 0, sizeof(*stats));
+    collect_stats(e, stats);
+    stats->d2h_bytes = d2h;
+  }
+  return B2A_OK;
+}
+
+extern "C" {
+
+int32_t b2a_score_batch(b2a_engine* e, int32_t mode, const b2a_scoring* scoring, const b2a_pairs* pairs,
+                        b2a_score_results* results, b2a_stats* stats) {
+  if (!e || !scoring || !pairs) return B2A_E_INVALID;
+  int32_t rc;
+  if (e->pipe_chunks >= 2 && results && pairs->n_pairs >= 262144) {  // as b2a_align_batch
+    e->staged = e->ran = false;
+    if (cudaSetDevice(e->device) != cudaSuccess) return e->fail(B2A_E_NO_DEVICE, "cudaSetDevice failed");
+    rc = align_batch_pipelined(e, mode, scoring, pairs, nullptr, results, stats);
+  } else {
+    rc = batch_stage(e, mode, scoring, pairs, true);
+    if (rc == B2A_OK) rc = b2a_batch_run(e);
+    if (rc == B2A_OK) rc = score_fetch(e, results, stats);
+  }
+  // the scratch now holds no traceback and no ops: nothing for b2a_batch_fetch / the record and compact calls
+  e->staged = e->ran = false;
+  return rc;
 }
 
 static int32_t banded_impl(b2a_engine* e, int32_t mode, const b2a_scoring* s, uint32_t k, uint32_t w,

@@ -207,6 +207,7 @@ B2A_HD void column_step(const LaneCtx<G>& c, const int32_t j, const int32_t tste
   constexpr bool PR = (FLAGS & F_PACKREL) != 0;  // packed keys with relative indices (see F_PACKREL): here like PK,
   constexpr bool PK = (FLAGS & F_PACKTRK) != 0 || PR;  // the caller passes chunk- / strip-relative cj and rowbase
   constexpr bool RELU = (FLAGS & F_RELU) != 0;
+  constexpr bool NOTB = (FLAGS & F_NOTB) != 0;
   constexpr bool TMASK = MASKED && !LUT;  // the column tracker has to skip the padded rows explicitly
   // S travels between cells as "S + open": So_d = S4 + go4d feeds the D chain of the next column and (as
   // the diagonal input) M of the next column, whose LUT/compare scores are pre-biased by -go4d; the I chain
@@ -248,10 +249,13 @@ B2A_HD void column_step(const LaneCtx<G>& c, const int32_t j, const int32_t tste
     }
     s4 = sP & ~3;
     // nibble = code | iext << 2 | dext << 3 = (sP - s4) + min(i4 - iop, 4) + 2 * min(d4 - dop, 4),
-    // accumulated as tbacc*16 + nibble (the oldest nibble falls off the top)
-    const int32_t fi = addmin(i4, -iop, 4), fd = addmin(d4, -dop, 4);
-    const int32_t nib = fmad(fd, k2, fi) + sP - s4;
-    tbacc[r] = (uint32_t)(fmad((int32_t)tbacc[r], k16, fmad(fd, k2, fi)) + sP - s4);
+    // accumulated as tbacc*16 + nibble (the oldest nibble falls off the top); score-only: column n's nibble only
+    int32_t nib = 0;
+    if (!NOTB || LAST) {
+      const int32_t fi = addmin(i4, -iop, 4), fd = addmin(d4, -dop, 4);
+      nib = fmad(fd, k2, fi) + sP - s4;
+      if (!NOTB) tbacc[r] = (uint32_t)(fmad((int32_t)tbacc[r], k16, fmad(fd, k2, fi)) + sP - s4);
+    }
     if (TC) {
       if (PK) {
         if (TMASK) {
@@ -313,6 +317,7 @@ B2A_HD void run_strip(const LaneCtx<G>& c, const int32_t s) {
   constexpr bool LUT = (FLAGS & F_LUT) != 0;
   constexpr bool PR = (FLAGS & F_PACKREL) != 0;
   constexpr bool PK = (FLAGS & F_PACKTRK) != 0 || PR;  // packed keys in the lanes (PR: relative indices)
+  constexpr bool NOTB = (FLAGS & F_NOTB) != 0;
   constexpr int P = 32 / G;
   constexpr int TBW = tbw_of(R);
   const int32_t m = c.m, n = c.n;
@@ -503,7 +508,7 @@ B2A_HD void run_strip(const LaneCtx<G>& c, const int32_t s) {
       in_i = iup;
       in_tv = Tv;
       in_ti = Ti;
-    } else {
+    } else if (!NOTB) {
 #pragma unroll
       for (int r = 0; r < R; ++r) tbacc[r] <<= 4;
     }
@@ -519,7 +524,7 @@ B2A_HD void run_strip(const LaneCtx<G>& c, const int32_t s) {
         }
       }
     }
-    if ((t & 7) == 7) {
+    if (!NOTB && (t & 7) == 7) {
       uint4* dst = tbs + (size_t)(t >> 3) * TBW * 32 + c.lane;
 #pragma unroll
       for (int qd = 0; qd < TBW; ++qd) {

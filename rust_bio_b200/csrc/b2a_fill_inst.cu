@@ -45,8 +45,10 @@ cudaError_t go(const FillParams& prm, uint32_t ntasks, int num_sms, cudaStream_t
 cudaError_t B2A_CAT(launch_fill_, B2A_G, B2A_R)(int flags, const FillParams& prm, uint32_t ntasks,
                                                 int num_sms, cudaStream_t stream, int* grid_out, int dry) {
   constexpr int ALL = F_TRACK_ROWS | F_TRACK_COLS | F_CLIPX;
-#define B2A_CASE(F) \
-  case (F): return go<(F)>(prm, ntasks, num_sms, stream, grid_out, dry);
+  // every variant twice: with the traceback, and score-only (F_NOTB, b2a_score_batch)
+#define B2A_CASE(F)                                                         \
+  case (F): return go<(F)>(prm, ntasks, num_sms, stream, grid_out, dry);   \
+  case (F) | F_NOTB: return go<(F) | F_NOTB>(prm, ntasks, num_sms, stream, grid_out, dry);
   switch (flags) {
     B2A_CASE(0)
     B2A_CASE(F_TRACK_ROWS)

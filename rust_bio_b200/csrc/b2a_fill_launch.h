@@ -30,8 +30,8 @@ B2A_DECLARE_FILL(8, 20)
 B2A_DECLARE_FILL(32, 8)
 B2A_DECLARE_FILL(32, 16)
 
-// the pair-packed 1x16 local fill (b2a_fill_pair16.cuh): two blocks per warp-task, int16x2 cells
-cudaError_t launch_fill_pair16(const FillParams& prm, int32_t bias, int num_sms, cudaStream_t stream, int* grid_out,
-                               int dry);
+// the pair-packed 1x16 local fill (b2a_fill_pair16.cuh): two blocks per warp-task, int16x2 cells; notb: score-only
+cudaError_t launch_fill_pair16(const FillParams& prm, int32_t bias, bool notb, int num_sms, cudaStream_t stream,
+                               int* grid_out, int dry);
 
 }  // namespace b2a

@@ -4,9 +4,11 @@
 
 namespace b2a {
 
-cudaError_t launch_fill_pair16(const FillParams& prm, int32_t bias, int num_sms, cudaStream_t stream, int* grid_out,
-                               int dry) {
-  auto kern = fill_pair16_kernel<16>;
+namespace {
+
+template <bool NOTB>
+cudaError_t go(const FillParams& prm, int32_t bias, int num_sms, cudaStream_t stream, int* grid_out, int dry) {
+  auto kern = fill_pair16_kernel<16, NOTB>;
   constexpr int WARPS = 4;
   const size_t smem = 64 + p16_lut_smem_bytes(prm.sc.alpha) + (size_t)WARPS * prm.smem_seq_bytes;
   cudaError_t err = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -28,6 +30,13 @@ cudaError_t launch_fill_pair16(const FillParams& prm, int32_t bias, int num_sms,
   if (grid_out) *grid_out = (int)grid;
   kern<<<grid, WARPS * 32, smem, stream>>>(prm, bias);
   return cudaGetLastError();
+}
+
+}  // namespace
+
+cudaError_t launch_fill_pair16(const FillParams& prm, int32_t bias, bool notb, int num_sms, cudaStream_t stream,
+                               int* grid_out, int dry) {
+  return notb ? go<true>(prm, bias, num_sms, stream, grid_out, dry) : go<false>(prm, bias, num_sms, stream, grid_out, dry);
 }
 
 }  // namespace b2a

@@ -146,8 +146,9 @@ struct P16Ctx {
   int32_t bias;
 };
 
-// one column of this lane's R rows (see column_step in b2a_fill.cuh for the cell it mirrors)
-template <int R, bool MASKED, bool LAST>
+// one column of this lane's R rows (see column_step in b2a_fill.cuh for the cell it mirrors); NOTB: score-only
+// (F_NOTB), no nibble accumulators -- column n's nibbles (the rows arena) are still computed
+template <int R, bool MASKED, bool LAST, bool NOTB>
 B2A_HD void p16_column(const P16Ctx& c, const int32_t j, const int32_t q4, const int32_t rowbase, const int32_t rv,
                        uint32_t (&Sp)[R], uint32_t (&Dp)[R], uint32_t (&SnR)[R], uint32_t (&acc)[R],
                        const int32_t (&xc)[R], const int32_t (&kcol)[R], const int32_t kmul, const uint32_t sdiag,
@@ -173,13 +174,18 @@ B2A_HD void p16_column(const P16Ctx& c, const int32_t j, const int32_t q4, const
     const uint32_t s4 = sP & 0xfffcfffcu;
     // ext flags: min(I4 - open, 4), min(D4 - open, 4) as min(open + 4, X4) - open; nibble =
     // code + iext*4 + dext*8 = (sP - s4) + (fi - iop) + 2*(fd - dop), exact per half (see the header)
-    const uint32_t fi = p16_addmin(iop, FOUR2, i4), fd = p16_addmin(dop, FOUR2, d4);
-    const int32_t fsum = fmad((int32_t)fd, k2, (int32_t)fi);
-    const int32_t osum = fmad((int32_t)dop, k2, (int32_t)iop);
-    const int32_t code = fmad((int32_t)s4, mone, (int32_t)sP);
-    int32_t a = fmad((int32_t)acc[r], kmul, fsum);
-    a = fmad(osum, mone, a);
-    acc[r] = (uint32_t)fmad(code, one, a);
+    int32_t fsum = 0, osum = 0, code = 0;
+    if (!NOTB || LAST) {
+      const uint32_t fi = p16_addmin(iop, FOUR2, i4), fd = p16_addmin(dop, FOUR2, d4);
+      fsum = fmad((int32_t)fd, k2, (int32_t)fi);
+      osum = fmad((int32_t)dop, k2, (int32_t)iop);
+      code = fmad((int32_t)s4, mone, (int32_t)sP);
+    }
+    if (!NOTB) {
+      int32_t a = fmad((int32_t)acc[r], kmul, fsum);
+      a = fmad(osum, mone, a);
+      acc[r] = (uint32_t)fmad(code, one, a);
+    }
     // column tracker: local key 256*S + (255 - r), two rows per 3-input max
     const uint32_t key = (uint32_t)fmad((int32_t)s4, k64, kcol[r]);
     if (r & 1) Tl = p16_umax3(Tl, key_even, key);
@@ -221,7 +227,7 @@ B2A_HD void p16_column(const P16Ctx& c, const int32_t j, const int32_t q4, const
 B2A_HD int32_t p16_key32(uint32_t k16) { return (int32_t)((k16 >> 8) << 12) + 3839 + (int32_t)(k16 & 255u); }
 
 // One strip (rows s*R+1 .. (s+1)*R) of this lane's two pairs.
-template <int R, bool MASKED>
+template <int R, bool MASKED, bool NOTB>
 B2A_HD void p16_strip(const P16Ctx& c, const int32_t s) {
   constexpr int TBW = tbw_of(R);
   const int32_t m = c.m, n = c.n, alpha = c.sc.alpha, B = c.bias;
@@ -292,10 +298,10 @@ B2A_HD void p16_strip(const P16Ctx& c, const int32_t s) {
       }
       uint32_t sup = in_s, iup = in_i, Tv = in_t;
       if (j == n) {
-        p16_column<R, MASKED, true>(c, j, q4, rowbase, rv, Sp, Dp, SnR, acc, xc, kcol, kmul, sup_prev, sup, iup, Tv,
+        p16_column<R, MASKED, true, NOTB>(c, j, q4, rowbase, rv, Sp, Dp, SnR, acc, xc, kcol, kmul, sup_prev, sup, iup, Tv,
                                     cap_s, cap_i);
       } else {
-        p16_column<R, MASKED, false>(c, j, q4, rowbase, rv, Sp, Dp, SnR, acc, xc, kcol, kmul, sup_prev, sup, iup, Tv,
+        p16_column<R, MASKED, false, NOTB>(c, j, q4, rowbase, rv, Sp, Dp, SnR, acc, xc, kcol, kmul, sup_prev, sup, iup, Tv,
                                      cap_s, cap_i);
       }
       sup_prev = in_s;
@@ -317,14 +323,14 @@ B2A_HD void p16_strip(const P16Ctx& c, const int32_t s) {
       in_s = sup;
       in_i = iup;
       in_t = Tv;
-    } else {
+    } else if (!NOTB) {
 #pragma unroll
       for (int r = 0; r < R; ++r) acc[r] = (uint32_t)fmad((int32_t)acc[r], kmul, 0);
     }
-    if ((t & 7) == 3) {
+    if (!NOTB && (t & 7) == 3) {
 #pragma unroll
       for (int r = 0; r < R; ++r) acc_hi[r] = acc[r];  // columns 0-3 of the group: the word's top 16 bits
-    } else if ((t & 7) == 7) {
+    } else if (!NOTB && (t & 7) == 7) {
       uint4* da = c.tb_a + (size_t)s * c.K * TBW * 32 + (size_t)(t >> 3) * TBW * 32 + c.lane;
       uint4* db = c.tb_b + (size_t)s * c.K * TBW * 32 + (size_t)(t >> 3) * TBW * 32 + c.lane;
 #pragma unroll
@@ -356,11 +362,11 @@ B2A_HD void p16_strip(const P16Ctx& c, const int32_t s) {
   }
 }
 
-template <int R>
+template <int R, bool NOTB = false>
 B2A_HD void p16_fill_lane(const P16Ctx& c) {
   for (int32_t s = 0; s < c.nstrips; ++s) {
-    if ((s + 1) * R <= c.m - 1) p16_strip<R, false>(c, s);
-    else p16_strip<R, true>(c, s);
+    if ((s + 1) * R <= c.m - 1) p16_strip<R, false, NOTB>(c, s);
+    else p16_strip<R, true, NOTB>(c, s);
   }
 }
 
@@ -368,7 +374,7 @@ B2A_HD void p16_fill_lane(const P16Ctx& c) {
 
 // Persistent kernel: a warp-task is a pair of blocks (2k, 2k+1) of the wave; y of both is staged by bulk copy,
 // x is read from global memory once per strip.
-template <int R>
+template <int R, bool NOTB>
 __global__ void __launch_bounds__(128, B2A_MINB) fill_pair16_kernel(const FillParams prm, const int32_t bias) {
   extern __shared__ __align__(128) uint8_t smem[];
   constexpr int WARPS = 4;
@@ -430,7 +436,7 @@ __global__ void __launch_bounds__(128, B2A_MINB) fill_pair16_kernel(const FillPa
     while (!mbar_try_wait(bar, parity)) {
     }
     parity ^= 1u;
-    p16_fill_lane<R>(c);
+    p16_fill_lane<R, NOTB>(c);
     __syncwarp();
   }
 }

@@ -35,8 +35,10 @@ struct Plan {
 
 inline uint64_t align_up(uint64_t v, uint64_t a) { return (v + a - 1) / a * a; }
 
+// score_only: the plan of a score-only batch (K1 with F_NOTB): no traceback arena, so the budget never closes a
+// wave -- the batch is one wave
 inline void build_plan(Plan& p, const uint32_t* x_len, const uint32_t* y_len, uint64_t n_pairs, int G,
-                       int R, uint64_t tb_budget) {
+                       int R, uint64_t tb_budget, bool score_only = false) {
   p.G = G;
   p.R = R;
   p.n_pairs = n_pairs;
@@ -96,7 +98,8 @@ inline void build_plan(Plan& p, const uint32_t* x_len, const uint32_t* y_len, ui
     const uint64_t bnd = align_up((uint64_t)(k.maxn + 1) * 32 * 16, 256);
     const uint64_t rows = align_up((uint64_t)ROWS_ARRAYS * k.rows_pad * 32 * 4, 256);
     const uint64_t rowm = align_up((uint64_t)(k.maxn + 1) * 32 * 2, 256);
-    const uint64_t tb = align_up((uint64_t)G * k.nstrips * k.K * TBW * 512, 256);
+    const uint64_t tb_raw = score_only ? 0 : (uint64_t)G * k.nstrips * k.K * TBW * 512;
+    const uint64_t tb = align_up(tb_raw, 256);
     if (b > w.block_lo && w.tb_bytes + tb > tb_budget) {  // close the wave
       w.block_hi = b;
       p.waves.push_back(w);
@@ -116,7 +119,7 @@ inline void build_plan(Plan& p, const uint32_t* x_len, const uint32_t* y_len, ui
     w.rows_bytes += rows;
     w.rowm_bytes += rowm;
     w.tb_bytes += tb;
-    p.total_tb += (uint64_t)G * k.nstrips * k.K * TBW * 512;
+    p.total_tb += tb_raw;
   }
   if (nblocks) {
     w.block_hi = nblocks;

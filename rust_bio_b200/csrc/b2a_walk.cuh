@@ -1089,64 +1089,109 @@ B2A_HD void walk_pair_coop(const int lane, const PairView& v, const bool filter_
   walk_finish(es, w, out);
 }
 
-#if defined(__CUDACC__)
+// ---------------------------------------------------------------------------------------------------------
+// Score-only K2 (b2a_score_batch): score, xend and yend without the interior traceback (K1 ran with F_NOTB).
+// score is S(m, n) after the fix-ups, which finish_matrix_* compute from what K1 leaves without the traceback.
+// xend / yend change only on TB_XCLIP_SUFFIX / TB_YCLIP_SUFFIX, and those codes live only in row m and column n;
+// the walk's (i, j) never increases, so once it stands on a cell with i < m and j < n neither can change again.
+// end_walk() is walk_run's state machine restricted to row m and column n: it stops at the first move that leaves
+// them (a prefix clip included), BEFORE it resolves the next layer -- the two LAZY resolutions that read an interior
+// nibble, INS out of row m and DEL out of column n, are such moves.  It flags the pair (status 1) on walk_run's
+// conditions met on that stretch; a reference panic deeper inside the matrix is not seen (the pair keeps the
+// fill's score and status 0).
+struct EndOut {
+  int32_t score;
+  uint32_t xend, yend, status;
+};
 
-// K2 for one pair (lane) of a block
-__device__ __forceinline__ void walk_lane(const WalkParams& prm, const Block& blk, const int lane) {
-  if ((uint32_t)lane >= blk.npairs) return;
-  const uint32_t sp = blk.first + lane;
-  const int32_t P = 32 / prm.G;
-  PairView v;
-  v.sc = prm.sc;
-  v.lut = prm.lut;
-  v.P = P;
-  v.m = (int32_t)prm.pm[sp];
-  v.n = (int32_t)prm.pn[sp];
-  v.pi = lane;
-  v.set_shape(prm.G, prm.R);
-  v.nstrips = (int32_t)blk.nstrips;
-  v.K = (int32_t)blk.K;
-  v.sub = lane / P;
-  v.g = lane % P;
-  v.packtrk = prm.packtrk;
-  v.maxn = (int32_t)blk.maxn;
-  v.bnd_base = bnd_index(prm.G, 0, lane, v.maxn);
-  v.bnd_stride = (int32_t)(bnd_index(prm.G, 1, lane, v.maxn) - v.bnd_base);
-  const uint32_t* seqw = reinterpret_cast<const uint32_t*>(prm.seq + blk.seq_off);
-  v.xw = seqw + (size_t)v.sub * blk.xwords * P + v.g;
-  v.yw = seqw + (size_t)prm.G * blk.xwords * P + (size_t)v.sub * blk.ywords * P + v.g;
-  v.bnd = reinterpret_cast<const int4*>(prm.bnd + blk.bnd_off);
-  v.rows = reinterpret_cast<int32_t*>(prm.rows + blk.rows_off);
-  v.rows_pad = (int32_t)blk.rows_pad;
-  v.rowm = reinterpret_cast<uint16_t*>(prm.rowm + blk.rowm_off);
-  v.tb = reinterpret_cast<const uint32_t*>(prm.tb + blk.tb_off);
-  const uint32_t cap = blk.maxm + blk.maxn + 4;
-  uint8_t* ops_end = prm.ops_scratch + blk.ops_off + (size_t)(lane + 1) * cap;
-  WalkOut o;
-  walk_pair(v, prm.filter_clips != 0, ops_end, o);
-  if (o.status) {  // the reference panics on this pair (mod.rs:905): no alignment is reported for it
-    o.score = MIN_SCORE;
-    o.n_ops = 0;
-    o.xstart = o.xend = o.ystart = o.yend = 0;
-    o.clip[0] = o.clip[1] = o.clip[2] = o.clip[3] = 0;
+B2A_HD void end_walk(const PairView& v, const EndState& es, const bool filter_clips, EndOut& out) {
+  const DevScoring& sc = v.sc;
+  const int32_t m = v.m, n = v.n;
+  const uint32_t cmN = es.cmN;
+  auto get_cell_n = [&](int32_t i) -> uint32_t { return (i == m) ? cmN : (uint32_t)v.row(ROWS_NL, i); };
+  auto get_s = [&](int32_t i, int32_t j) -> uint32_t {  // (i, j) in row m or column n (walk_run's order of cases)
+    if (j == n) return cell_s(get_cell_n(i));
+    if (i == 0) return row0_sbits(sc, j, n);  // m == 0: K2 keeps no row-m cells
+    return cell_s((uint32_t)v.rowm[j * 32 + v.pi]);
+  };
+  int32_t i = m, j = n, guard = m + n + 8;
+  uint32_t layer = cell_s(cmN), xend = (uint32_t)m, yend = (uint32_t)n, status = 0, nclip = 0;
+  while (layer != TB_START) {
+    if (--guard < 0) {
+      status = 1;
+      break;
+    }
+    uint32_t next = 0;
+    bool lazy = true;  // the next layer is S of the cell the move lands on
+    if (layer == TB_INS) {
+      if (j == n) {
+        next = cell_i(get_cell_n(i));
+        lazy = false;
+      } else {
+        next = cell_i((uint32_t)v.rowm[j * 32 + v.pi]);  // i == m
+        lazy = next == LAZY;
+      }
+      i -= 1;
+    } else if (layer == TB_DEL) {
+      if (i == 0 || i == m) {
+        next = (i == 0) ? row0_dbits(sc, j) : cell_d((uint32_t)v.rowm[j * 32 + v.pi]);
+        lazy = false;
+      } else {
+        next = cell_d(get_cell_n(i));  // j == n
+        lazy = next == LAZY;
+      }
+      j -= 1;
+    } else if (layer == TB_MATCH || layer == TB_SUBST) {
+      i -= 1;
+      j -= 1;
+    } else if (layer == TB_XCLIP_PREFIX) {
+      if (!filter_clips) ++nclip;
+      i = 0;
+    } else if (layer == TB_XCLIP_SUFFIX) {
+      int32_t lx;
+      if (j == n) lx = es.LxN;
+      else if (j == 0) lx = es.Lx0;
+      else lx = (m >= 2) ? m - decode_boundary(v.load_bnd(j), v.packtrk != 0, sc.xclip_suffix, m).Ti : 0;
+      if (!filter_clips) ++nclip;
+      i -= lx;
+      xend = (uint32_t)i;
+    } else if (layer == TB_YCLIP_PREFIX) {
+      if (!filter_clips) ++nclip;
+      j = 0;
+    } else if (layer == TB_YCLIP_SUFFIX) {
+      int32_t ly;
+      if (i == m) ly = es.Lym;
+      else if (i == 0 || n == 0) ly = n;
+      else ly = n - v.row(ROWS_LY, i);
+      if (!filter_clips) ++nclip;
+      j -= ly;
+      yend = (uint32_t)j;
+    } else {
+      status = 1;  // panic!("Dint expect this!") mod.rs:905
+      break;
+    }
+    if (i < 0 || j < 0) {
+      status = 1;
+      break;
+    }
+    if (i != m && j != n) break;  // left row m and column n: xend and yend are final
+    layer = lazy ? get_s(i, j) : next;
   }
-  const uint32_t dst = prm.order[sp];
-  prm.score[dst] = o.score;
-  prm.xstart[dst] = o.xstart;
-  prm.xend[dst] = o.xend;
-  prm.ystart[dst] = o.ystart;
-  prm.yend[dst] = o.yend;
-  prm.n_ops[dst] = o.n_ops;
-  prm.ops_src[dst] = blk.ops_off + (uint64_t)(lane + 1) * cap - o.n_ops;
-  prm.status[dst] = o.status;
-  if (o.status) atomicOr(prm.err_flag, 1u);
-#pragma unroll
-  for (int k = 0; k < 4; ++k) prm.clip_len[4 * (size_t)dst + k] = o.clip[k];
+  if (nclip > 4) status = 1;  // walk_finish: a lower bound of the full walk's clip count
+  out.score = es.SmN;
+  out.xend = xend;
+  out.yend = yend;
+  out.status = status;
+  if (status) {  // as walk_lane reports a pair the reference panics on
+    out.score = MIN_SCORE;
+    out.xend = out.yend = 0;
+  }
 }
 
-// K2, one warp per pair
-__device__ __forceinline__ void walk_warp(const WalkParams& prm, const Block& blk, const int pi, const int lane,
-                                          uint8_t* seq_smem) {
+#if defined(__CUDACC__)
+
+// the view K2 has of pair `pi` of a block
+__device__ __forceinline__ PairView pair_view(const WalkParams& prm, const Block& blk, const int pi) {
   const uint32_t sp = blk.first + pi;
   const int32_t P = 32 / prm.G;
   PairView v;
@@ -1173,16 +1218,57 @@ __device__ __forceinline__ void walk_warp(const WalkParams& prm, const Block& bl
   v.rows_pad = (int32_t)blk.rows_pad;
   v.rowm = reinterpret_cast<uint16_t*>(prm.rowm + blk.rowm_off);
   v.tb = reinterpret_cast<const uint32_t*>(prm.tb + blk.tb_off);
-  if (seq_smem) {  // this warp's slice of the CTA's dynamic shared memory: x bytes, then y bytes (word granules)
-    const int32_t xwn = (v.m + 3) >> 2, ywn = (v.n + 3) >> 2;
-    uint32_t* xs = reinterpret_cast<uint32_t*>(seq_smem);
-    uint32_t* ys = xs + ((blk.maxm + 3) >> 2);
-    for (int32_t w = lane; w < xwn; w += 32) xs[w] = v.xw[(size_t)w * P];
-    for (int32_t w = lane; w < ywn; w += 32) ys[w] = v.yw[(size_t)w * P];
-    __syncwarp();
-    v.xs8 = reinterpret_cast<const uint8_t*>(xs);
-    v.ys8 = reinterpret_cast<const uint8_t*>(ys);
+  return v;
+}
+
+// K2 for one pair (lane) of a block
+__device__ __forceinline__ void walk_lane(const WalkParams& prm, const Block& blk, const int lane) {
+  if ((uint32_t)lane >= blk.npairs) return;
+  const uint32_t sp = blk.first + lane;
+  const PairView v = pair_view(prm, blk, lane);
+  const uint32_t cap = blk.maxm + blk.maxn + 4;
+  uint8_t* ops_end = prm.ops_scratch + blk.ops_off + (size_t)(lane + 1) * cap;
+  WalkOut o;
+  walk_pair(v, prm.filter_clips != 0, ops_end, o);
+  if (o.status) {  // the reference panics on this pair (mod.rs:905): no alignment is reported for it
+    o.score = MIN_SCORE;
+    o.n_ops = 0;
+    o.xstart = o.xend = o.ystart = o.yend = 0;
+    o.clip[0] = o.clip[1] = o.clip[2] = o.clip[3] = 0;
   }
+  const uint32_t dst = prm.order[sp];
+  prm.score[dst] = o.score;
+  prm.xstart[dst] = o.xstart;
+  prm.xend[dst] = o.xend;
+  prm.ystart[dst] = o.ystart;
+  prm.yend[dst] = o.yend;
+  prm.n_ops[dst] = o.n_ops;
+  prm.ops_src[dst] = blk.ops_off + (uint64_t)(lane + 1) * cap - o.n_ops;
+  prm.status[dst] = o.status;
+  if (o.status) atomicOr(prm.err_flag, 1u);
+#pragma unroll
+  for (int k = 0; k < 4; ++k) prm.clip_len[4 * (size_t)dst + k] = o.clip[k];
+}
+
+// K2, one warp per pair
+// the pair's x and y copied into this warp's slice of the CTA's dynamic shared memory (x bytes, then y bytes)
+__device__ __forceinline__ void stage_pair_seqs(PairView& v, const Block& blk, const int lane, uint8_t* seq_smem) {
+  const int32_t P = v.P;
+  const int32_t xwn = (v.m + 3) >> 2, ywn = (v.n + 3) >> 2;
+  uint32_t* xs = reinterpret_cast<uint32_t*>(seq_smem);
+  uint32_t* ys = xs + ((blk.maxm + 3) >> 2);
+  for (int32_t w = lane; w < xwn; w += 32) xs[w] = v.xw[(size_t)w * P];
+  for (int32_t w = lane; w < ywn; w += 32) ys[w] = v.yw[(size_t)w * P];
+  __syncwarp();
+  v.xs8 = reinterpret_cast<const uint8_t*>(xs);
+  v.ys8 = reinterpret_cast<const uint8_t*>(ys);
+}
+
+__device__ __forceinline__ void walk_warp(const WalkParams& prm, const Block& blk, const int pi, const int lane,
+                                          uint8_t* seq_smem) {
+  const uint32_t sp = blk.first + pi;
+  PairView v = pair_view(prm, blk, pi);
+  if (seq_smem) stage_pair_seqs(v, blk, lane, seq_smem);
   const uint32_t cap = blk.maxm + blk.maxn + 4;
   uint8_t* ops_end = prm.ops_scratch + blk.ops_off + (size_t)(pi + 1) * cap;
   WalkOut o;
@@ -1208,6 +1294,39 @@ __device__ __forceinline__ void walk_warp(const WalkParams& prm, const Block& bl
   for (int k = 0; k < 4; ++k) prm.clip_len[4 * (size_t)dst + k] = o.clip[k];
 }
 
+__device__ __forceinline__ void score_store(const WalkParams& prm, const uint32_t sp, const EndOut& o) {
+  const uint32_t dst = prm.order[sp];
+  prm.score[dst] = o.score;
+  prm.xend[dst] = o.xend;
+  prm.yend[dst] = o.yend;
+  prm.status[dst] = o.status;
+  if (o.status) atomicOr(prm.err_flag, 1u);
+}
+
+// score-only K2 for one pair (lane) of a block: row m and the fix-ups, then the end walk
+__device__ __forceinline__ void score_lane(const WalkParams& prm, const Block& blk, const int lane) {
+  if ((uint32_t)lane >= blk.npairs) return;
+  const PairView v = pair_view(prm, blk, lane);
+  EndState es;
+  finish_matrix_seq(v, es);
+  EndOut o;
+  end_walk(v, es, prm.filter_clips != 0, o);
+  score_store(prm, blk.first + lane, o);
+}
+
+// score-only K2, one warp per pair: the cooperative row m and fix-ups, then lane 0's end walk
+__device__ __forceinline__ void score_warp(const WalkParams& prm, const Block& blk, const int pi, const int lane,
+                                           uint8_t* seq_smem) {
+  PairView v = pair_view(prm, blk, pi);
+  if (seq_smem) stage_pair_seqs(v, blk, lane, seq_smem);
+  EndState es;
+  finish_matrix_coop<32>(lane, v, es);
+  if (lane != 0) return;
+  EndOut o;
+  end_walk(v, es, prm.filter_clips != 0, o);
+  score_store(prm, blk.first + pi, o);
+}
+
 #if defined(B2A_DEFINE_WALK_KERNEL)  // one translation unit (b2a_engine.cu) owns the stand-alone kernel
 __global__ void __launch_bounds__(1024, 1) walk_warp_kernel(const WalkParams prm) {  // 64 registers; CTAs of 1..32 warps
   extern __shared__ __align__(16) uint8_t walk_smem[];  // seq_smem_per_warp bytes per warp, or none
@@ -1227,6 +1346,27 @@ __global__ void __launch_bounds__(128, 8) walk_kernel(const WalkParams prm) {
   if (gw >= prm.nblocks) return;
   const Block blk = prm.blocks[gw];
   walk_lane(prm, blk, lane);
+}
+
+// score-only K2 in the two forms of walk_warp_kernel / walk_kernel
+__global__ void __launch_bounds__(1024, 1) score_warp_kernel(const WalkParams prm) {
+  extern __shared__ __align__(16) uint8_t walk_smem[];
+  const uint32_t gw = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  const uint32_t b = gw >> 5, pi = gw & 31u;
+  if (b >= prm.nblocks) return;
+  const Block blk = prm.blocks[b];
+  if (pi >= blk.npairs) return;
+  uint8_t* mine = prm.seq_smem_per_warp ? walk_smem + (size_t)(threadIdx.x >> 5) * prm.seq_smem_per_warp : nullptr;
+  score_warp(prm, blk, (int)pi, lane, mine);
+}
+
+__global__ void __launch_bounds__(128, 8) score_kernel(const WalkParams prm) {
+  const uint32_t gw = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  if (gw >= prm.nblocks) return;
+  const Block blk = prm.blocks[gw];
+  score_lane(prm, blk, lane);
 }
 #endif
 

@@ -7,7 +7,7 @@ from typing import Dict, Optional, Tuple
 import numpy as np
 
 from . import _lib
-from ._lib import B2AError, CPairs, CResults, CScoring, CStats
+from ._lib import B2AError, CPairs, CResults, CScoreResults, CScoring, CStats
 
 Batch = Tuple[np.ndarray, np.ndarray, np.ndarray, np.ndarray, np.ndarray]
 
@@ -66,6 +66,23 @@ class Results:
 
     def as_dict(self):
         return {k: getattr(self, k) for k in ("score", "xstart", "xend", "ystart", "yend")}
+
+
+class ScoreResults:
+    """Host outputs of one score-only batch: score, xend, yend (numpy arrays), and per-pair B2A_PAIR_* codes when
+    requested with pair_status=True (else a pair on which the reference would panic fails the whole batch)."""
+
+    def __init__(self, n_pairs: int, pair_status: bool = False):
+        self.n_pairs = n_pairs
+        self.score = np.zeros(n_pairs, dtype=np.int32)
+        self.xend = np.zeros(n_pairs, dtype=np.uint32)
+        self.yend = np.zeros(n_pairs, dtype=np.uint32)
+        self.status = np.zeros(max(1, n_pairs), dtype=np.uint32) if pair_status else None
+        p = lambda a: a.ctypes.data_as(C.c_void_p)
+        self.c = CScoreResults(p(self.score), p(self.xend), p(self.yend), p(self.status) if pair_status else None)
+
+    def as_dict(self):
+        return {k: getattr(self, k) for k in ("score", "xend", "yend")}
 
 
 class Engine:
@@ -139,6 +156,16 @@ class Engine:
         cp = self._cpairs(batch)
         self._check(self._L.b2a_align_batch(self._h, int(mode), C.byref(cscoring), C.byref(cp),
                                             C.byref(results.c), C.byref(self.stats)))
+        return results
+
+    def score_batch(self, mode: int, cscoring: CScoring, batch: Batch,
+                    results: Optional[ScoreResults] = None) -> ScoreResults:
+        """b2a_score_batch: score, xend and yend of every pair without the traceback (host buffers in and out)."""
+        if results is None:
+            results = ScoreResults(len(batch[2]))
+        cp = self._cpairs(batch)
+        self._check(self._L.b2a_score_batch(self._h, int(mode), C.byref(cscoring), C.byref(cp), C.byref(results.c),
+                                            C.byref(self.stats)))
         return results
 
     def align_batch_banded(self, mode: int, cscoring: CScoring, k: int, w: int, batch: Batch,

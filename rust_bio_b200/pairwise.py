@@ -17,7 +17,7 @@ import numpy as np
 from . import scores as _scores
 from ._lib import (CScoring, MIN_SCORE, MODE_CUSTOM, MODE_GLOBAL, MODE_LOCAL, MODE_SEMIGLOBAL)
 from .alignment import Alignment, AlignmentMode, AlignmentOperation
-from .engine import Engine, Results, default_engine, pack_pairs
+from .engine import Engine, Results, ScoreResults, default_engine, pack_pairs
 
 __all__ = ["MIN_SCORE", "MatchParams", "Scoring", "Aligner", "MatchFunc"]
 
@@ -249,6 +249,51 @@ class Aligner:
 
     def local_batch(self, pairs, on_panic: str = "raise"):
         return self._batch(MODE_LOCAL, pairs, on_panic)
+
+    # score-only batch forms: (score, xend, yend) of the Alignment the batch forms above return, without the
+    # traceback (b2a_score_batch) -- for callers that rank or filter candidates and never read the path
+    def _scores_batch(self, mode: int, pairs: Sequence[Tuple[bytes, bytes]],
+                      on_panic: str = "raise") -> List[Optional[Tuple[int, int, int]]]:
+        """on_panic as in the batch forms.  A pair is flagged only where the reference's panic lies on the part
+        of the walk the score-only call replays (row m and column n, include/b200align.h)."""
+        from ._lib import B2AError
+        batch = pack_pairs(pairs)
+        cs, keep = self.scoring.to_c(batch)
+        res = self.engine.score_batch(mode, cs, batch, results=ScoreResults(len(pairs), pair_status=True))
+        out = []
+        for i in range(len(pairs)):
+            st = int(res.status[i])
+            if st:
+                if on_panic == "raise":
+                    raise B2AError(-4, f"pair {i}: " + _PAIR_STATUS_TEXT.get(st, str(st)))
+                out.append(None)
+                continue
+            out.append((int(res.score[i]), int(res.xend[i]), int(res.yend[i])))
+        return out
+
+    def custom_scores_batch(self, pairs, on_panic: str = "raise"):
+        return self._scores_batch(MODE_CUSTOM, pairs, on_panic)
+
+    def global_scores_batch(self, pairs, on_panic: str = "raise"):
+        return self._scores_batch(MODE_GLOBAL, pairs, on_panic)
+
+    def semiglobal_scores_batch(self, pairs, on_panic: str = "raise"):
+        return self._scores_batch(MODE_SEMIGLOBAL, pairs, on_panic)
+
+    def local_scores_batch(self, pairs, on_panic: str = "raise"):
+        return self._scores_batch(MODE_LOCAL, pairs, on_panic)
+
+    def custom_score(self, x: bytes, y: bytes) -> Tuple[int, int, int]:
+        return self._scores_batch(MODE_CUSTOM, [(x, y)])[0]
+
+    def global_score(self, x: bytes, y: bytes) -> Tuple[int, int, int]:
+        return self._scores_batch(MODE_GLOBAL, [(x, y)])[0]
+
+    def semiglobal_score(self, x: bytes, y: bytes) -> Tuple[int, int, int]:
+        return self._scores_batch(MODE_SEMIGLOBAL, [(x, y)])[0]
+
+    def local_score(self, x: bytes, y: bytes) -> Tuple[int, int, int]:
+        return self._scores_batch(MODE_LOCAL, [(x, y)])[0]
 
     # per-pair forms, mod.rs:591, 925, 954, 986
     def custom(self, x: bytes, y: bytes) -> Alignment:

@@ -66,8 +66,23 @@ pub mod alignment {
             clip_len: *mut u32,
             status: *mut u32, // per-pair B2A_PAIR_* codes; null = a failing pair fails the batch (-> panic, like the reference)
         }
+        #[repr(C)]
+        struct b2a_score_results {
+            score: *mut i32,
+            xend: *mut u32,
+            yend: *mut u32,
+            status: *mut u32,
+        }
         #[link(name = "b200align")]
         extern "C" {
+            fn b2a_score_batch(
+                e: *mut c_void,
+                mode: i32,
+                scoring: *const b2a_scoring,
+                pairs: *const b2a_pairs,
+                results: *mut b2a_score_results,
+                stats: *mut c_void,
+            ) -> i32;
             fn b2a_engine_create(out: *mut *mut c_void, device_id: i32) -> i32;
             // every visible GPU from this one process (include/b200align.h: b2a_multi_*)
             fn b2a_multi_create(out: *mut *mut c_void, device_ids: *const i32, n_devices: i32) -> i32;
@@ -476,6 +491,78 @@ pub mod alignment {
                     })
                     .collect()
             }
+
+            /// Score-only batch (b2a_score_batch): (score, xend, yend) of the Alignment `batch` returns, without the
+            /// traceback.  Panics where the reference would on the part of the walk it replays (include/b200align.h).
+            pub(crate) fn scores(&mut self, mode: i32, pairs: &[(&[u8], &[u8])]) -> Vec<(i32, usize, usize)> {
+                let n = pairs.len();
+                let (mut x_off, mut y_off, mut x_len, mut y_len) = (Vec::with_capacity(n), Vec::with_capacity(n), Vec::with_capacity(n), Vec::with_capacity(n));
+                let mut blob: Vec<u8> = Vec::new();
+                let mut present = [false; 256];
+                for (x, y) in pairs {
+                    for (s, off) in [(x, &mut x_off), (y, &mut y_off)] {
+                        while blob.len() % 16 != 0 {
+                            blob.push(0);
+                        }
+                        off.push(blob.len() as u64);
+                        blob.extend_from_slice(s);
+                        for &b in s.iter() {
+                            present[b as usize] = true;
+                        }
+                    }
+                    x_len.push(x.len() as u32);
+                    y_len.push(y.len() as u32);
+                }
+                let alphabet: Vec<u8> = (0..=255u8).filter(|b| present[*b as usize]).collect();
+                let mut table = vec![0i32; 256 * 256];
+                for &a in &alphabet {
+                    for &b in &alphabet {
+                        table[a as usize * 256 + b as usize] = self.scoring.match_fn.score(a, b);
+                    }
+                }
+                let (ms, mm) = self.scoring.match_scores.unwrap_or((0, 0));
+                let cs = b2a_scoring {
+                    gap_open: self.scoring.gap_open,
+                    gap_extend: self.scoring.gap_extend,
+                    xclip_prefix: self.scoring.xclip_prefix,
+                    xclip_suffix: self.scoring.xclip_suffix,
+                    yclip_prefix: self.scoring.yclip_prefix,
+                    yclip_suffix: self.scoring.yclip_suffix,
+                    match_score: ms,
+                    mismatch_score: mm,
+                    has_match_scores: self.scoring.match_scores.is_some() as i32,
+                    table: table.as_ptr(),
+                    alphabet: alphabet.as_ptr(),
+                    alphabet_len: alphabet.len() as u32,
+                };
+                let cp = b2a_pairs {
+                    seq_blob: blob.as_ptr(),
+                    x_off: x_off.as_ptr(),
+                    x_len: x_len.as_ptr(),
+                    y_off: y_off.as_ptr(),
+                    y_len: y_len.as_ptr(),
+                    blob_bytes: blob.len() as u64,
+                    n_pairs: n as u64,
+                };
+                let (mut score, mut xe, mut ye) = (vec![0i32; n], vec![0u32; n], vec![0u32; n]);
+                let mut res = b2a_score_results {
+                    score: score.as_mut_ptr(),
+                    xend: xe.as_mut_ptr(),
+                    yend: ye.as_mut_ptr(),
+                    status: std::ptr::null_mut(),
+                };
+                let rc = unsafe { b2a_score_batch(self.engine, mode, &cs, &cp, &mut res, std::ptr::null_mut()) };
+                if rc != 0 {
+                    let msg = unsafe { CStr::from_ptr(b2a_last_error(self.engine)) }.to_string_lossy().into_owned();
+                    panic!("{}", msg);
+                }
+                (0..n).map(|p| (score[p], xe[p] as usize, ye[p] as usize)).collect()
+            }
+
+            pub fn custom_scores_batch(&mut self, pairs: &[(&[u8], &[u8])]) -> Vec<(i32, usize, usize)> { self.scores(0, pairs) }
+            pub fn global_scores_batch(&mut self, pairs: &[(&[u8], &[u8])]) -> Vec<(i32, usize, usize)> { self.scores(1, pairs) }
+            pub fn semiglobal_scores_batch(&mut self, pairs: &[(&[u8], &[u8])]) -> Vec<(i32, usize, usize)> { self.scores(2, pairs) }
+            pub fn local_scores_batch(&mut self, pairs: &[(&[u8], &[u8])]) -> Vec<(i32, usize, usize)> { self.scores(3, pairs) }
 
             pub fn custom_batch(&mut self, pairs: &[(&[u8], &[u8])]) -> Vec<Alignment> { self.batch(0, None, pairs) }
             pub fn global_batch(&mut self, pairs: &[(&[u8], &[u8])]) -> Vec<Alignment> { self.batch(1, None, pairs) }
